@@ -342,7 +342,7 @@ def run_e2e(ctx, dfd, n, args):
     schema = batches[0].schema
     times = []
     st = None
-    for it in range(2 + max(1, args.steps // 2)):
+    for it in range(2 + args.steps):
         ex = dfd.RepartitionExec(ctx, schema, dfd.Partitioning.Hash([0], NUM_PARTITIONS), chunk_rows=args.e2e_chunk_rows,
                                  pipeline_depth=3, pinned_pool_chunks=args.e2e_pool_chunks)
         readers = [ex.execute(p) for p in range(NUM_PARTITIONS)]
@@ -387,6 +387,30 @@ def run_e2e(ctx, dfd, n, args):
                          "pinned_chunks_reused": int(st["pinned_chunks_reused"]), "push_ms": st["ns_push"] / 1e6,
                          "wait_d2h_ms": st["ns_wait_d2h"] / 1e6, "wait_pool_ms": st["ns_wait_pool"] / 1e6},
             "pcie": pcie, "frac_of_pcie_duplex": pcie_frac}
+
+
+DUMP_SAMPLE_ROWS = 1 << 18  # rows sampled by --dump-outputs: 17 float64 arrays of 2 MiB (36 MB) stay under 64 MB
+
+
+def dump_outputs(out_dir, torch, outs, starts, counts):
+    """Write what the last timed step handed its caller, so that two builds can be compared output for output:
+    `partition_counts` (rows per destination) and, for a fixed seeded sample of positions in destination order
+    (`sample_positions`; destination p is rows [starts[p], starts[p] + counts[p]) of every output column), each
+    int64 output column as `col<c>_hi` / `col<c>_lo`, its signed high and unsigned low 32 bits in float64, which
+    round-trip exactly.  Every array is float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(counts.sum())
+    rng = np.random.Generator(np.random.PCG64(20261017))
+    pos = np.arange(n) if n <= DUMP_SAMPLE_ROWS else np.sort(rng.choice(n, DUMP_SAMPLE_ROWS, replace=False))
+    first = np.concatenate([[0], np.cumsum(counts)])
+    dest = np.searchsorted(first, pos, side="right") - 1
+    idx = torch.from_numpy(starts[dest] + (pos - first[dest])).to(outs[0].device)
+    arrays = {"partition_counts": counts, "sample_positions": pos}
+    for c, col in enumerate(outs):
+        v = col.index_select(0, idx).cpu().numpy()
+        arrays[f"col{c}_hi"], arrays[f"col{c}_lo"] = v >> 32, v & 0xFFFFFFFF
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
 
 
 TRAFFIC_ONEPASS = 8.564484e9  # dram__bytes_read.sum + dram__bytes_write.sum of one k_scatter_onepass launch at cfg-2 (profiles/r02c_ncu_summary.md)
@@ -595,7 +619,7 @@ def run_multi_gpu(args, torch, dfd, world):
         n_chunks = max(2, min(16, n // (1 << 20)))
         e2e_times = []
         got = 0
-        for it in range(2 + max(1, args.steps // 2)):
+        for it in range(2 + args.steps):
             dist.barrier()
             t0 = time.perf_counter()
             cps = node.shuffle_host(ex, h_in, n, n_chunks, h_out, cap)
@@ -664,7 +688,13 @@ def main():
                     help="cfg2 = the BASELINE.json headline (default; what the driver runs); cfg3/4/5 = the other configs (bench_workloads.py)")
     ap.add_argument("--kernel", default="onepass", choices=["onepass", "twopass"],
                     help="1-GPU partition path: single-pass k_scatter<ONEPASS> (regions) or K1/K1b/K2 (dense)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of the last step's "
+                    "outputs as DIR/<name>.npy (float64; cfg2 on one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "cfg2" or args.gpus != 1):
+        ap.error("--dump-outputs covers the cfg2 workload on one GPU")
     if args.impl == "reference":
         if args.workload == "cfg4":
             import bench_workloads
@@ -729,9 +759,17 @@ def main():
         ms_total = ctx.timer_stop()
     m = ctx.metrics()
     if onepass:
-        _, counts = part.collect()
+        starts, counts = part.collect()
         assert int(counts.sum()) == n and ctx.metrics()["onepass_reruns"] == 0, "a destination region overflowed inside the timed loop"
     ctx.set_profiling(False)
+    if args.dump_outputs:
+        if not onepass:  # dense layout: destination p is rows [part_starts[p], part_starts[p + 1])
+            from datafusion_distributed_b200 import _native as nv
+
+            bounds = np.empty(NUM_PARTITIONS + 1, dtype=np.int64)
+            nv.check(nv.lib().dfd_memcpy_d2h(ctx.handle, bounds.ctypes.data, part.part_starts_device_ptr(), bounds.nbytes))
+            starts, counts = bounds[:-1], np.diff(bounds)
+        dump_outputs(args.dump_outputs, torch, outs, starts, counts)
     ms_per_step = ms_total / args.steps
     value = n / (ms_per_step / 1e3)
 
