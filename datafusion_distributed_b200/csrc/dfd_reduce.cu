@@ -6,12 +6,15 @@
 // aggregate states there shrinks what crosses the network.  Here the partitioned table is already on the GPU
 // (output of dfd_partition_device), so the merge runs on it in place of a PCIe round trip:
 //   k_group_insert   open-addressing table of REPRESENTATIVE ROW indices (one u32 per slot): a row claims an empty slot
-//                    with atomicCAS or joins the group whose representative has equal key bytes (any number / width of
-//                    fixed-width keys — the keys themselves are never copied into the table)
+//                    with atomicCAS or joins the group whose representative has equal key bytes AND lies in the same
+//                    input partition (any number / width of fixed-width keys — the keys themselves are never copied into
+//                    the table).  Groups never cross partitions: the caller's part_starts need not follow the group keys.
 //   k_group_count    groups per destination partition (representatives only)      -> exclusive scan (host, N+1 values)
 //   k_group_place    every group gets an output row inside its partition; key columns copied, states initialised
 //   k_group_combine  every input row folds its states into its group's output row with atomics
-//                    (SUM i64 / f64 / i128 (two 64-bit adds with carry), MIN / MAX i64 / f64)
+//                    (SUM i64 / f64 / i128 (two 64-bit adds with carry), MIN / MAX i64, MIN / MAX f64 in the integer
+//                    image of IEEE-754 totalOrder, so the result is the same whatever order the atomics land in)
+//   k_group_finish   only with a float MIN / MAX column: maps those states back from the totalOrder image to doubles
 // Integer / byte work; random access into an L2-resident table for the cardinalities PartialReduce is used for.
 #include <cuda_runtime.h>
 
@@ -101,16 +104,28 @@ __device__ __forceinline__ uint32_t partition_of(const int64_t* starts, uint32_t
     return lo;
 }
 
+// Bit pattern of a double <-> an int64 whose signed order is IEEE-754 totalOrder (Rust's f64::total_cmp):
+// -NaN < -inf < ... < -0.0 < +0.0 < ... < +inf < +NaN.  Negative values get their 63 low bits flipped; the map is its own
+// inverse.  MIN / MAX of these integers is an exact fold, so float MIN / MAX states do not depend on the atomics' order.
+__device__ __forceinline__ long long f64_total_order(long long b) {
+    return b ^ (long long)((unsigned long long)(b >> 63) >> 1);
+}
+
 __global__ void __launch_bounds__(256) k_group_insert(const __grid_constant__ ReduceParams P) {
     for (int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; row < P.n_rows; row += (int64_t)gridDim.x * blockDim.x) {
-        uint32_t s = (uint32_t)key_hash(P, row) & P.table_mask;
+        // the row's input partition is [lo, hi): only a representative inside it can be the row's group
+        const uint32_t p = partition_of(P.part_starts, P.N, row);
+        const int64_t lo = p == 0 ? 0 : P.part_starts[p];
+        const int64_t hi = p + 1 == P.N ? P.n_rows : P.part_starts[p + 1];
+        // the partition shifts the start slot, so equal keys of different partitions do not share a probe chain
+        uint32_t s = (uint32_t)(key_hash(P, row) + (uint64_t)p * 0x9e3779b97f4a7c15ULL) & P.table_mask;
         for (;;) {
             uint32_t rep = P.table[s];
             if (rep == SLOT_EMPTY) {
                 rep = atomicCAS(P.table + s, SLOT_EMPTY, (uint32_t)row);
                 if (rep == SLOT_EMPTY) break;  // this row represents a new group
             }
-            if (keys_equal(P, (int64_t)rep, row)) break;
+            if ((int64_t)rep >= lo && (int64_t)rep < hi && keys_equal(P, (int64_t)rep, row)) break;
             s = (s + 1) & P.table_mask;
         }
         P.row_slot[row] = s;
@@ -130,8 +145,9 @@ __device__ __forceinline__ void state_init(const ReduceCol& c, char* dst) {
         case DFD_AGG_SUM_I128: ((uint64_t*)dst)[0] = 0; ((uint64_t*)dst)[1] = 0; break;
         case DFD_AGG_MIN_I64: *(long long*)dst = 0x7fffffffffffffffLL; break;
         case DFD_AGG_MAX_I64: *(long long*)dst = (long long)0x8000000000000000ULL; break;
-        case DFD_AGG_MIN_F64: *(double*)dst = __longlong_as_double(0x7ff0000000000000LL); break;   // +inf
-        case DFD_AGG_MAX_F64: *(double*)dst = __longlong_as_double((long long)0xfff0000000000000ULL); break;  // -inf
+        // float MIN / MAX states live in the totalOrder image until k_group_finish
+        case DFD_AGG_MIN_F64: *(long long*)dst = 0x7fffffffffffffffLL; break;
+        case DFD_AGG_MAX_F64: *(long long*)dst = (long long)0x8000000000000000ULL; break;
     }
 }
 
@@ -155,25 +171,6 @@ __global__ void __launch_bounds__(256) k_group_place(const __grid_constant__ Red
     }
 }
 
-__device__ __forceinline__ void atomic_min_f64(double* addr, double v) {
-    unsigned long long* a = (unsigned long long*)addr;
-    unsigned long long old = *a;
-    while (v < __longlong_as_double((long long)old)) {
-        const unsigned long long prev = atomicCAS(a, old, (unsigned long long)__double_as_longlong(v));
-        if (prev == old) break;
-        old = prev;
-    }
-}
-__device__ __forceinline__ void atomic_max_f64(double* addr, double v) {
-    unsigned long long* a = (unsigned long long*)addr;
-    unsigned long long old = *a;
-    while (v > __longlong_as_double((long long)old)) {
-        const unsigned long long prev = atomicCAS(a, old, (unsigned long long)__double_as_longlong(v));
-        if (prev == old) break;
-        old = prev;
-    }
-}
-
 __global__ void __launch_bounds__(256) k_group_combine(const __grid_constant__ ReduceParams P) {
     for (int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; row < P.n_rows; row += (int64_t)gridDim.x * blockDim.x) {
         const int64_t o = (int64_t)P.slot_out[P.row_slot[row]];
@@ -187,8 +184,8 @@ __global__ void __launch_bounds__(256) k_group_combine(const __grid_constant__ R
                 case DFD_AGG_SUM_F64: atomicAdd((double*)dst, *(const double*)src); break;
                 case DFD_AGG_MIN_I64: atomicMin((long long*)dst, *(const long long*)src); break;
                 case DFD_AGG_MAX_I64: atomicMax((long long*)dst, *(const long long*)src); break;
-                case DFD_AGG_MIN_F64: atomic_min_f64((double*)dst, *(const double*)src); break;
-                case DFD_AGG_MAX_F64: atomic_max_f64((double*)dst, *(const double*)src); break;
+                case DFD_AGG_MIN_F64: atomicMin((long long*)dst, f64_total_order(*(const long long*)src)); break;
+                case DFD_AGG_MAX_F64: atomicMax((long long*)dst, f64_total_order(*(const long long*)src)); break;
                 case DFD_AGG_SUM_I128: {
                     // two's complement 128-bit add as two 64-bit atomics: each add propagates its OWN carry exactly once
                     const unsigned long long lo = ((const unsigned long long*)src)[0], hi = ((const unsigned long long*)src)[1];
@@ -198,6 +195,17 @@ __global__ void __launch_bounds__(256) k_group_combine(const __grid_constant__ R
                     break;
                 }
             }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) k_group_finish(const __grid_constant__ ReduceParams P, int64_t n_out) {
+    for (int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; o < n_out; o += (int64_t)gridDim.x * blockDim.x) {
+        for (int c = 0; c < P.n_cols; ++c) {
+            const ReduceCol& col = P.col[c];
+            if (col.op != DFD_AGG_MIN_F64 && col.op != DFD_AGG_MAX_F64) continue;
+            long long* dst = (long long*)(col.out + o * 8);
+            *dst = f64_total_order(*dst);
         }
     }
 }
@@ -282,6 +290,13 @@ extern "C" int dfd_partial_reduce_device(dfd_ctx* c, const dfd_column* in_cols, 
     k_group_combine<<<grid, 256, 0, s>>>(P);
     if ((e = cudaGetLastError()) != cudaSuccess) return cuda_error(e, "k_group_place / k_group_combine");
     c->metrics.kernel_launches += 4;
+    bool float_min_max = false;
+    for (int i = 0; i < n_cols; ++i) float_min_max |= agg_ops[i] == DFD_AGG_MIN_F64 || agg_ops[i] == DFD_AGG_MAX_F64;
+    if (float_min_max) {
+        k_group_finish<<<grid, 256, 0, s>>>(P, out_part_starts_host[N]);
+        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_error(e, "k_group_finish");
+        c->metrics.kernel_launches += 1;
+    }
     if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return cuda_error(e, "partial reduce");  // (out_part_starts_host is caller memory)
     return DFD_OK;
 }

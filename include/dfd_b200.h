@@ -431,7 +431,19 @@ int dfd_exchange_phase_ms(dfd_exchange* x, double* out3, uint64_t* n_shuffles);
  * per distinct key, partition p = rows [out_part_starts[p], out_part_starts[p+1]) of out_cols (capacity n_rows; row order
  * inside a partition is unspecified, like a hash aggregate's).  Feed it to dfd_exchange_gather(DFD_ROUTE_SHUFFLE) — the
  * rows never leave the GPU between Partial aggregation, repartition, PartialReduce and the exchange.
- * Fixed-width non-null keys and states (nullable group keys / states: DFD_ERR_UNSUPPORTED).  Synchronous. */
+ * Fixed-width non-null keys and states (nullable group keys / states: DFD_ERR_UNSUPPORTED).  Synchronous.
+ * Semantics (tests/test_reduce_exact_gpu.py):
+ *   - Groups never cross input partitions: a row joins a group only if its key bytes are equal AND it lies in the same
+ *     input partition, so the same key in two partitions is two groups, each in its own output partition, whatever
+ *     decided part_starts.  Key equality is byte equality (float keys: to_bits equality; +0.0, -0.0 and every NaN
+ *     payload are distinct groups).
+ *   - SUM_I64 and SUM_I128 wrap (two's complement, mod 2^64 / 2^128); MIN / MAX_I64 are exact.
+ *   - MIN / MAX_F64 follow IEEE-754 totalOrder (Rust's f64::total_cmp): -NaN < -inf < ... < -0.0 < +0.0 < ... < +inf
+ *     < +NaN.  The result is bit-identical to a sequential fold in any row order (an all-NaN group gives a NaN; a group
+ *     of +0.0 and -0.0 gives -0.0 / +0.0).  Parity unpinned: DataFusion's MIN / MAX groups accumulator is not in this
+ *     repository, so agreement with its float order is not checked (DESIGN.md §2).
+ *   - SUM_F64 is the only result that is not bit-exact: the additions land in an unspecified order, and for a group of
+ *     k finite rows |result - exact sum| <= (k-1) * 2^-53 * sum|x|.  A NaN row, or +inf with -inf, gives NaN. */
 typedef enum {
     DFD_AGG_SUM_I64 = 0,  /* also COUNT states */
     DFD_AGG_SUM_F64 = 1,
