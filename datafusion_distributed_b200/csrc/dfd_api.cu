@@ -589,6 +589,17 @@ int dfd::launch_lengths_to_offsets(const void* len, int ow, int64_t n, unsigned 
     return DFD_OK;
 }
 
+int dfd::launch_var_gather(const void* in_off, int ow, int64_t in_offset, const uint8_t* in_data, const uint32_t* src, const void* out_off,
+                           uint8_t* out_data, int64_t n, cudaStream_t s) {
+    if (n <= 0) return DFD_OK;
+    const int64_t blocks = (n + 255) / 256;
+    const unsigned grid = (unsigned)(blocks > 0x7fffffffLL ? 0x7fffffffLL : blocks);
+    if (ow == 8) k_var_copy_bytes<int64_t, true><<<grid, 256, 0, s>>>((const int64_t*)in_off, in_offset, in_data, src, (const int64_t*)out_off, out_data, n);
+    else k_var_copy_bytes<int32_t, true><<<grid, 256, 0, s>>>((const int32_t*)in_off, in_offset, in_data, src, (const int32_t*)out_off, out_data, n);
+    LAUNCH_CHECK("k_var_copy_bytes");
+    return DFD_OK;
+}
+
 int dfd::partition_device_locked(Partitioner* p, const dfd_column* in_cols, int n_cols, int64_t n_rows,
                                  const dfd_column* out_cols, cudaStream_t stream, bool var_bytes_known) {
     PartitionJob job;

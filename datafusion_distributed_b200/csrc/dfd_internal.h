@@ -126,6 +126,10 @@ int launch_bytes_to_bits(const uint8_t* in, int64_t n, void* out_words, cudaStre
 int launch_offsets_to_lengths(const void* off, int ow, int64_t n, void* len, cudaStream_t s);
 int launch_var_dest_bytes(const void* off, int ow, const int64_t* part_starts, uint32_t N, int64_t* bytes, int64_t* first, cudaStream_t s);
 int launch_lengths_to_offsets(const void* len, int ow, int64_t n, unsigned long long* block_sums /*[n/2048 + 2]*/, void* out_off, cudaStream_t s);
+// out_data[out_off[j], out_off[j+1]) <- in_data at input row src[j] (+ in_offset), n output rows: k_var_copy_bytes with the
+// lengths taken from the output offsets (a row may be shorter in the output than in the input, e.g. a null written as "").
+int launch_var_gather(const void* in_off, int ow, int64_t in_offset, const uint8_t* in_data, const uint32_t* src, const void* out_off,
+                      uint8_t* out_data, int64_t n, cudaStream_t s);
 
 // Aligned write-out (k_scatter KV > K) is used for the peer-store exchange at small N (measured: +15% over NVLink, -5% local).
 bool use_aligned(uint32_t N, bool peer);

@@ -1195,8 +1195,9 @@ __global__ void __launch_bounds__(VAR_BLOCK) k_var_write_offsets(const OFF* __re
 // row's (source offset, length, destination offset) — the three dependent loads src -> offsets -> bytes, 32 rows in flight
 // per warp — then the warp copies the non-empty rows one after the other with all 32 lanes on consecutive bytes, so both
 // the loads and the stores of a string are coalesced whatever its length (a thread-per-row byte loop is neither, and a
-// warp runs as long as its longest string).
-template <typename OFF>
+// warp runs as long as its longest string).  LEN_FROM_OUT takes each row's length from the OUTPUT offsets instead, so that a
+// row whose output slot is shorter than its source (PartialReduce: a null key written as length 0) copies only that many.
+template <typename OFF, bool LEN_FROM_OUT = false>
 __global__ void __launch_bounds__(256) k_var_copy_bytes(const OFF* __restrict__ in_off, int64_t in_offset,
                                                          const uint8_t* __restrict__ in_data, const uint32_t* __restrict__ src,
                                                          const OFF* __restrict__ out_off, uint8_t* __restrict__ out_data, int64_t n) {
@@ -1208,8 +1209,8 @@ __global__ void __launch_bounds__(256) k_var_copy_bytes(const OFF* __restrict__ 
         if (j < n) {
             const int64_t r = (int64_t)src[j] + in_offset;
             so = (int64_t)in_off[r];
-            len = (int64_t)in_off[r + 1] - so;
             dof = (int64_t)out_off[j];
+            len = LEN_FROM_OUT ? (int64_t)out_off[j + 1] - dof : (int64_t)in_off[r + 1] - so;
         }
         unsigned todo = __ballot_sync(0xffffffffu, len > 0);
         while (todo) {

@@ -141,7 +141,13 @@ class HashPartitioner:
 class PartialReduceExec:
     """≙ AggregateExec(mode = PartialReduce) above the producers' hash RepartitionExec
     (src/distributed_planner/partial_reduce_below_network_shuffles.rs:17-100): merges rows with equal group keys inside
-    each destination partition of a partitioned device table (`dfd_partial_reduce_device`)."""
+    each destination partition of a partitioned device table (`dfd_partial_reduce_device`).
+
+    Group keys may be fixed-width, Boolean, Utf8, LargeUtf8 or Binary columns, and keys and states may be nullable: NULL
+    is a group value, null states are skipped, and a state is null when every input state of its group is.  An output
+    column is nullable iff its `validity` is set; the default outputs (`DeviceColumn.empty_like`) get a validity bitmap
+    exactly when the input column has one, and string outputs a byte capacity equal to the input's byte count, which
+    the reduced keys never exceed."""
 
     def __init__(self, ctx: WorkerContext, key_cols: Sequence[int], agg_ops: Sequence[int]):
         """agg_ops[c] = nv.AGG_* for state column c, -1 for the group-key columns."""

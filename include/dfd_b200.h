@@ -431,19 +431,41 @@ int dfd_exchange_phase_ms(dfd_exchange* x, double* out3, uint64_t* n_shuffles);
  * per distinct key, partition p = rows [out_part_starts[p], out_part_starts[p+1]) of out_cols (capacity n_rows; row order
  * inside a partition is unspecified, like a hash aggregate's).  Feed it to dfd_exchange_gather(DFD_ROUTE_SHUFFLE) — the
  * rows never leave the GPU between Partial aggregation, repartition, PartialReduce and the exchange.
- * Fixed-width non-null keys and states (nullable group keys / states: DFD_ERR_UNSUPPORTED).  Synchronous.
- * Semantics (tests/test_reduce_exact_gpu.py):
- *   - Groups never cross input partitions: a row joins a group only if its key bytes are equal AND it lies in the same
+ * Synchronous.
+ * Columns: group keys are fixed-width (1 / 2 / 4 / 8 / 16 bytes), Boolean (bit-packed; the Arrow offset is a bit offset) or
+ * Utf8 / LargeUtf8 / Binary; aggregate states are fixed-width.  Keys and states may be nullable.  out_cols[c] has the
+ * kind (and offset width) of in_cols[c]; an op on a Boolean or string column, a kind / offset-width mismatch, and
+ * Dictionary or view columns give DFD_ERR_UNSUPPORTED.
+ * Nullability: a column is nullable iff out_cols[c].validity != NULL (the convention of dfd_shuffle_device_onepass).  A
+ * nullable input needs an output validity bitmap (DFD_ERR_UNSUPPORTED otherwise); a non-null input with an output bitmap
+ * gets every bit set.  Bit-packed outputs (validity, Boolean key values) follow dfd_partition_device: 4-byte aligned,
+ * ceil(n_rows / 32) * 4 bytes, output offset 0; the library zeroes them itself and writes them with 32-bit atomic ORs.
+ * String keys: out_cols[c].offsets gets n_out + 1 entries of the input's offset width and out_cols[c].values the
+ * representatives' bytes in output-row order, so partition p is the zero-copy slice [out_part_starts[p],
+ * out_part_starts[p+1]) as in dfd_partition_device.  out_cols[c].values_bytes is the byte capacity: if it is smaller than
+ * the group keys' bytes the call returns DFD_ERR_CAPACITY with the needed size in the message and writes no output column.
+ * n_rows == 0 writes offsets[0] = 0 of every string output.
+ * Semantics (tests/test_reduce_exact_gpu.py, tests/test_reduce_nullable_gpu.py):
+ *   - Groups never cross input partitions: a row joins a group only if its keys are equal AND it lies in the same
  *     input partition, so the same key in two partitions is two groups, each in its own output partition, whatever
- *     decided part_starts.  Key equality is byte equality (float keys: to_bits equality; +0.0, -0.0 and every NaN
- *     payload are distinct groups).
+ *     decided part_starts.  Fixed-width key equality is byte equality (float keys: to_bits equality; +0.0, -0.0 and every
+ *     NaN payload are distinct groups).  String keys are equal iff their lengths and bytes are; Boolean keys by value.
+ *   - NULL is a group value, as in SQL GROUP BY: the NULLs of a key column are equal to each other and differ from every
+ *     non-null value (an empty string and NULL are two groups); with several keys the null pattern is part of the key.
+ *     The bytes under a null key are never read.  A null key is written as zero bytes (a string: length 0, a Boolean: 0).
+ *   - Null input states are skipped; an output state is null iff every input state of its group is null, and is then
+ *     written as 0.  The value bytes of a null input state never reach the result.
  *   - SUM_I64 and SUM_I128 wrap (two's complement, mod 2^64 / 2^128); MIN / MAX_I64 are exact.
  *   - MIN / MAX_F64 follow IEEE-754 totalOrder (Rust's f64::total_cmp): -NaN < -inf < ... < -0.0 < +0.0 < ... < +inf
  *     < +NaN.  The result is bit-identical to a sequential fold in any row order (an all-NaN group gives a NaN; a group
- *     of +0.0 and -0.0 gives -0.0 / +0.0).  Parity unpinned: DataFusion's MIN / MAX groups accumulator is not in this
- *     repository, so agreement with its float order is not checked (DESIGN.md §2).
+ *     of +0.0 and -0.0 gives -0.0 / +0.0).
+ *   - Parity unpinned: DataFusion's groups accumulators (MIN / MAX, and the null handling of every op) are not in this
+ *     repository, so agreement with their float order and null semantics is not checked (DESIGN.md §2).
  *   - SUM_F64 is the only result that is not bit-exact: the additions land in an unspecified order, and for a group of
- *     k finite rows |result - exact sum| <= (k-1) * 2^-53 * sum|x|.  A NaN row, or +inf with -inf, gives NaN. */
+ *     k finite rows |result - exact sum| <= (k-1) * 2^-53 * sum|x|.  A NaN row, or +inf with -inf, gives NaN.
+ * Kernel launches (dfd_metrics.kernel_launches) for n_rows > 0: 4 + F + 4 * S, where F = 1 if some state column is
+ * MIN / MAX_F64 or a MIN / MAX column with an input validity bitmap (the finishing pass), else 0, and S = the number of
+ * string key columns (a 3-launch lengths -> offsets scan and one byte gather each).  n_rows == 0 launches nothing. */
 typedef enum {
     DFD_AGG_SUM_I64 = 0,  /* also COUNT states */
     DFD_AGG_SUM_F64 = 1,
